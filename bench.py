@@ -8,6 +8,7 @@ candidates per request) x 256 requests = 8192 bands per GPU, i.e. a 629 MB H/b w
 
   python bench.py --gpus 1 --steps 5 --warmup 3                 # this framework
   python bench.py --impl reference --gpus 1 --steps 3 --warmup 1 # the reference's CPU path (oracle port, all host threads)
+  python bench.py --gpus 1 --steps 5 --warmup 3 --dump-outputs DIR  # + the last timed step's results as DIR/*.npy
 
 Prints ONE JSON line on rank 0 (see the contract in the task statement / DESIGN.md §6).
 """
@@ -46,7 +47,33 @@ def parse():
     ap.add_argument("--no-single-request", action="store_true")
     ap.add_argument("--total-bands", type=int, default=None, help="STRONG scaling: this many bands in total, split evenly over "
                     "the GPUs (BASELINE config 4: --workload C4 --total-bands 512 --gpus 4); overrides --requests")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="after the timed steps, write what the last one "
+                    "computed (bands, per-band cost / chi2 / status / LM iterations) as DIR/<name>.npy, float64, <= 64 MB")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, poses, per_band):
+    """--dump-outputs: the results a caller of the timed path receives, one DIR/<name>.npy (float64) per array, at most
+    DUMP_BYTES in all. Per-band results are written whole; the bands' poses too when they fit, else those of a fixed
+    seeded sample of bands. poses_bands.npy holds the indices of the bands in poses.npy. Pose rows at and past a band's
+    length n are not part of the result and are written as 0."""
+    os.makedirs(out_dir, exist_ok=True)
+    out = {k: np.asarray(v, dtype=np.float64) for k, v in per_band.items()}
+    B = poses.shape[0]
+    room = DUMP_BYTES - sum(v.nbytes for v in out.values()) - 8 * B - 4096 * (len(out) + 2)     # npy headers
+    keep = min(B, room // (8 * poses[0].size))
+    idx = np.arange(B) if keep == B else np.sort(np.random.default_rng(0).choice(B, keep, replace=False))
+    sel = np.array(poses[idx], dtype=np.float64)
+    sel[np.arange(sel.shape[1])[None, :] >= np.asarray(per_band["n"])[idx][:, None]] = 0.0
+    out["poses"], out["poses_bands"] = sel, idx.astype(np.float64)
+    for name, v in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), v)
 
 
 def make_workload(a, rank):
@@ -283,7 +310,10 @@ def run_reference(a, rank, world):
         return
     p, hb, args, desc, cand = make_workload(a, 0)
     reps = a.cpu_reps or max(20, a.steps)
-    cpu, _, _ = cpu_arm(p, hb, args, cand, a.workload, reps, max(1, a.warmup))
+    cpu, _, h = cpu_arm(p, hb, args, cand, a.workload, reps, max(1, a.warmup))
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, h.poses, {"n": h.n, "cost": h.cost, "chi2": h.chi2, "status": h.status,
+                                               "lm_iters": h.lm_iters})
     value = cpu["value"]
     line = {"impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": a.gpus, "steps": a.steps,
             "warmup": a.warmup, "ms_per_step": cpu["ms_per_rep"], "higher_is_better": True, "scaling": "weak",
@@ -371,6 +401,13 @@ def run_b200(a, rank, local_rank, world):
     if world > 1:
         dist.barrier()
     clocks = sampler.stop()
+    if a.dump_outputs and rank == 0:    # before the profiled pass below overwrites the results of the last timed step
+        like = lambda d, arr: d.cpu().numpy().view(arr.dtype).reshape(arr.shape)     # byte tensors -> host arrays
+        per_band = {"n": like(d_n, hb.n), "cost": d_cost.cpu().numpy(), "chi2": d_chi2.cpu().numpy(),
+                    "status": d_status.cpu().numpy(), "lm_iters": d_iters.cpu().numpy()}
+        if world > 1:
+            per_band["cost_all_ranks"] = d_all_cost.cpu().numpy()
+        dump_outputs(a.dump_outputs, like(d_poses, hb.poses), per_band)
     dev_ms = sum(s.elapsed_time(e) for s, e in ev)
     launches_per_step = g.launch_count()
     lm_iters_step = int(d_iters.sum().item())

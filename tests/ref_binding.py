@@ -3,21 +3,115 @@ src/timed_elastic_band.cpp, src/obstacles.cpp and the headers they include) comp
 oracle/ref_shims/ (Eigen / boost / ROS message stand-ins and a restated g2o optimizer). TEST INFRASTRUCTURE: it pins the
 oracle restatement; nothing in the product may load it.
 
-/root/reference exists only in the build container: the library is built there (`make -C oracle ref`, also done by
-__graft_entry__.build()) and travels to the GPU box as a prebuilt file; `available()` tells tests whether it is there."""
+The library can only be built next to the reference's sources (`make -C oracle ref`). The tests that pin against it
+read the reference's results from tests/golden/golden_pin_v1.npz through `Pins`; tests/golden/make_golden_pin.py
+records that file by running the same tests against the library."""
 import ctypes as C
+import hashlib
 import os
 import subprocess
 
 import numpy as np
+import pytest
 
 from teb_local_planner_b200 import abi
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 REF_SO = os.path.join(ROOT, "oracle", "_ref", "libteb_ref.so")
 REFERENCE_TREE = "/root/reference"
+GOLDEN_PIN = os.path.join(ROOT, "tests", "golden", "golden_pin_v1.npz")
+RECORD = None       # {key: Pins} while make_golden_pin.py records GOLDEN_PIN from the library
 
 _lib = None
+_golden = None
+
+
+def _leaves(x):
+    """a result as a flat list of float64 arrays: tuples / lists in order, complex as (re, im), -0.0 as 0.0"""
+    if isinstance(x, (tuple, list)):
+        return [a for y in x for a in _leaves(y)]
+    if isinstance(x, complex):
+        x = (x.real, x.imag)
+    return [np.asarray(x, dtype=np.float64) + 0.0]
+
+
+def digest(x):
+    """128-bit digest of a result's shapes and float64 bits (equal digests <=> np.array_equal on every leaf, for
+    results without NaN)"""
+    h = hashlib.sha256()
+    for a in _leaves(x):
+        h.update(np.array(a.shape, np.int64).tobytes())
+        h.update(np.ascontiguousarray(a).tobytes())
+    return h.digest()[:16]
+
+
+class Pins:
+    """The reference's results one test compares against, in call order. Bit-equality checks keep a digest of the
+    reference's result (the results of some tests run to hundreds of MB); tolerance checks keep the values, in float64
+    or, where the test allows for the rounding, float32."""
+    STREAMS = {np.dtype(np.float64): "/values", np.dtype(np.float32): "/values32"}
+
+    def __init__(self, key):
+        self.key, self.nd, self.nl = key, 0, 0
+        self.nv = dict.fromkeys(self.STREAMS.values(), 0)
+        if RECORD is not None:
+            self.digests, self.layout = [], []
+            self.values = {s: [] for s in self.STREAMS.values()}
+            RECORD[key] = self
+            return
+        global _golden
+        if _golden is None:
+            _golden = np.load(GOLDEN_PIN, allow_pickle=False)
+        get = lambda s: _golden[key + s] if key + s in _golden.files else np.zeros(0)
+        self.digests, self.layout = get("/digests"), get("/layout")
+        self.values = {s: get(s) for s in self.STREAMS.values()}
+
+    def equal(self, live, mine, what=""):
+        """assert that `mine` is bit equal to the reference's result `live()`"""
+        got = digest(mine)
+        if RECORD is not None:
+            self.digests.append(digest(live()))
+        assert self.nd < len(self.digests), f"{self.key}: no stored reference result #{self.nd} (make_golden_pin.py)"
+        want = bytes(self.digests[self.nd])
+        self.nd += 1
+        assert got == want, f"{self.key} #{self.nd - 1} {what}: differs from the reference's result"
+
+    def value(self, live, dtype=np.float64):
+        """the reference's result `live()` as a list of float64 arrays (see _leaves), stored as `dtype`"""
+        stream = self.STREAMS[np.dtype(dtype)]
+        if RECORD is not None:
+            leaves = [a.astype(dtype).astype(np.float64) for a in _leaves(live())]
+            self.layout += [len(leaves)] + [k for a in leaves for k in (a.ndim, *a.shape)]
+            self.values[stream] += [a.reshape(-1).astype(dtype) for a in leaves]
+            return leaves
+        assert self.nl < len(self.layout), f"{self.key}: no stored reference result (make_golden_pin.py)"
+        out, L = [], self.layout
+        count, self.nl = int(L[self.nl]), self.nl + 1
+        for _ in range(count):
+            nd = int(L[self.nl])
+            shape = tuple(int(s) for s in L[self.nl + 1:self.nl + 1 + nd])
+            self.nl += 1 + nd
+            size, at = int(np.prod(shape)), self.nv[stream]
+            out.append(self.values[stream][at:at + size].astype(np.float64).reshape(shape))
+            self.nv[stream] += size
+        return out
+
+    def arrays(self):
+        """what GOLDEN_PIN stores for this test"""
+        out = {}
+        if self.digests:
+            out[self.key + "/digests"] = np.frombuffer(b"".join(self.digests), np.uint8).reshape(-1, 16)
+        if self.layout:
+            out[self.key + "/layout"] = np.array(self.layout, np.int64)
+        for stream, vals in self.values.items():
+            if vals:
+                out[self.key + stream] = np.concatenate(vals)
+        return out
+
+
+@pytest.fixture
+def pins(request):
+    return Pins(f"{request.module.__name__.rsplit('.', 1)[-1]}::{request.node.name}")
 
 
 def build_ref():

@@ -6,7 +6,8 @@ TebOptimalPlanner) expose the same operation codes (teb_ref_band_op / teb_host_b
 Covers initTrajectoryToGoal (start / goal, plan, 2-D path of the graph search), updateAndPruneTEB,
 findClosestTrajectoryPose, the time / distance sums, isTrajectoryInsideRegion, autoResize, getVelocityCommand,
 getVelocityProfile and getFullTrajectory - the functions the round-1 review found lifted; they are rewritten and this is
-what keeps them equal to the reference in behaviour."""
+what keeps them equal to the reference in behaviour. The reference's results are digests in tests/golden/golden_pin_v1.npz
+(`ref_binding.Pins`), recorded from the library by tests/golden/make_golden_pin.py."""
 import ctypes as C
 import math
 import os
@@ -15,22 +16,27 @@ import numpy as np
 import pytest
 
 from tests import ref_binding as rb
+from tests.ref_binding import pins  # noqa: F401  (fixture)
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-pytestmark = pytest.mark.skipif(not rb.available(), reason="oracle/_ref/libteb_ref.so not built (needs /root/reference)")
+
+
+def _band_op(fn):
+    fn.restype = C.c_int32
+    fn.argtypes = [C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32]
+    return fn
 
 
 @pytest.fixture(scope="module")
-def ops():
+def host():
     from teb_local_planner_b200 import build as b
     b.build()
     b.build_host()
-    host = C.CDLL(b.HOST_PIN)
-    ref = rb.lib()
-    for fn in (host.teb_host_band_op, ref.teb_ref_band_op):
-        fn.restype = C.c_int32
-        fn.argtypes = [C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32]
+    return _band_op(C.CDLL(b.HOST_PIN).teb_host_band_op)
 
+
+@pytest.fixture
+def ops(host, pins):
     def run(fn, op, rec, args, cap=8192):
         rec = None if rec is None else np.ascontiguousarray(rec, dtype=np.float64)
         a = np.ascontiguousarray(args, dtype=np.float64)
@@ -40,11 +46,9 @@ def ops():
         return out[:k].copy()
 
     def both(op, rec, args):
-        h = run(host.teb_host_band_op, op, rec, args)
-        r = run(ref.teb_ref_band_op, op, rec, args)
-        assert len(h) == len(r), (op, len(h), len(r))
-        assert np.array_equal(h, r), (op, args, np.abs(h - r).max() if len(h) else None)
-        return r
+        h = run(host, op, rec, args)
+        pins.equal(lambda: run(_band_op(rb.lib().teb_ref_band_op), op, rec, args), h, (op, args))
+        return h
 
     return both
 

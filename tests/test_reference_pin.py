@@ -8,9 +8,11 @@ edge by edge (errors, information, Jacobians incl. the two analytic overrides), 
 updateAndPruneTEB. The bar is BIT EQUALITY (both sides are fp64, compiled without FMA contraction); where a libm call
 order differs the tolerance is written at the assertion.
 
-Runs wherever the library exists (it is built in the container that holds /root/reference and travels as a prebuilt
-file); the committed golden vectors generated from it (tests/golden/golden_ref_v1.npz) keep the oracle pinned elsewhere."""
+The reference's side of every comparison is read from tests/golden/golden_pin_v1.npz (`ref_binding.Pins`), recorded
+from the library by tests/golden/make_golden_pin.py: the values where a tolerance applies, a digest of the result where
+the bar is bit equality."""
 import ctypes as C
+import functools
 import os
 
 import numpy as np
@@ -19,39 +21,34 @@ import pytest
 from teb_local_planner_b200 import abi, scenes
 from tests import ref_binding as rb
 from tests import scenarios
+from tests.ref_binding import pins  # noqa: F401  (fixture)
 
-pytestmark = pytest.mark.skipif(not rb.available(), reason="oracle/_ref/libteb_ref.so not built (needs /root/reference)")
 GOLDEN_REF = os.path.join(os.path.dirname(__file__), "golden", "golden_ref_v1.npz")
 
 
-def test_default_params_are_the_reference_constructor_defaults(teblib):
-    ref = rb.default_params()
+def test_default_params_are_the_reference_constructor_defaults(teblib, pins):
+    names = [name for name, _ in abi.TebParams._fields_ if not name.startswith("_")]
+    field = lambda q, name: list(getattr(q, name)) if isinstance(getattr(q, name), C.Array) else getattr(q, name)
+    ref = pins.value(lambda: [np.array(field(rb.default_params(), name)) for name in names])
     mine = abi.default_params()
     lib = abi.TebParams()
     teblib.tebgpu_default_params(C.byref(lib))
-    for name, _ in abi.TebParams._fields_:
-        if name.startswith("_"):
-            continue
-        a, b, c = getattr(ref, name), getattr(mine, name), getattr(lib, name)
-        if isinstance(a, C.Array):
-            assert list(a) == list(b) == list(c), name
-        else:
-            assert a == b == c, name
+    for name, a in zip(names, ref):
+        assert np.array_equal(a, field(mine, name)) and np.array_equal(a, field(lib, name)), name
 
 
-def test_penalties_bit_equal(oracle):
+def test_penalties_bit_equal(oracle, pins):
     L = oracle.lib()
     rng = np.random.default_rng(0)
     vals = np.concatenate([rng.normal(0, 1, 4000), [0.0, 0.35, -0.35, 0.4, -0.4, 0.45, 0.05, -0.05, 0.5, 0.55, 0.6]])
-    for v in vals:
-        for a, eps in ((0.4, 0.05), (0.3, 0.0), (0.5, 0.05)):
-            assert L.teb_oracle_penalty_interval(v, a, eps) == rb.penalty(0, v, a, 0.0, eps)
-            assert L.teb_oracle_penalty_interval2(v, -0.2, a, eps) == rb.penalty(1, v, -0.2, a, eps)
-            assert L.teb_oracle_penalty_below(v, a, eps) == rb.penalty(2, v, a, 0.0, eps)
+    for a, eps in ((0.4, 0.05), (0.3, 0.0), (0.5, 0.05)):
+        pins.equal(lambda: [[rb.penalty(0, v, a, 0.0, eps), rb.penalty(1, v, -0.2, a, eps), rb.penalty(2, v, a, 0.0, eps)] for v in vals],
+                   [[L.teb_oracle_penalty_interval(v, a, eps), L.teb_oracle_penalty_interval2(v, -0.2, a, eps),
+                     L.teb_oracle_penalty_below(v, a, eps)] for v in vals], (a, eps))
 
 
 @pytest.mark.parametrize("footprint", ["point", "circular", "two_circles", "line", "polygon"])
-def test_distances_every_footprint_and_obstacle_type(oracle, footprint):
+def test_distances_every_footprint_and_obstacle_type(oracle, pins, footprint):
     p, hb = scenarios.scenario("shapes_" + footprint, candidates=2)
     obst = hb.obstacles[0][:hb.obst_count[0]]
     kinds = set(int(o["type"]) for o in obst)
@@ -59,18 +56,18 @@ def test_distances_every_footprint_and_obstacle_type(oracle, footprint):
     circ = obst[0].copy()
     circ["type"], circ["radius"] = abi.TEB_OBST_CIRCULAR, 0.3
     rng = np.random.default_rng(5)
-    worst = 0.0
+    queries = []
     for o in list(obst) + [circ]:
         if not o["dynamic"]:            # a static obstacle has no velocity in the reference (obstacles.h:206 sets both)
             o = o.copy()
             o["vx"], o["vy"] = 0.0, 0.0
         for _ in range(12):
             pose = np.array([o["x"] + rng.normal(0, 1.0), o["y"] + rng.normal(0, 1.0), rng.uniform(-np.pi, np.pi)])
-            for t in (None, 0.0, 1.7):
-                d_ref = rb.distance(p, pose, o, hb.obst_vertices[0], t)
-                d_orc = oracle.distance(p, pose, o, hb.obst_vertices[0], 0.0 if t is None else t) if (t is not None) else \
-                    _static_distance(oracle, p, pose, o, hb.obst_vertices[0])
-                worst = max(worst, abs(d_ref - d_orc))
+            queries += [(pose, o, t) for t in (None, 0.0, 1.7)]
+    d_ref = pins.value(lambda: [rb.distance(p, pose, o, hb.obst_vertices[0], t) for pose, o, t in queries])
+    d_orc = [oracle.distance(p, pose, o, hb.obst_vertices[0], 0.0 if t is None else t) if (t is not None) else
+             _static_distance(oracle, p, pose, o, hb.obst_vertices[0]) for pose, o, t in queries]
+    worst = np.abs(np.array(d_ref) - np.array(d_orc)).max()
     assert worst <= 1e-15, worst
 
 
@@ -82,7 +79,7 @@ def _static_distance(oracle, p, pose, o, verts):
 
 
 @pytest.mark.parametrize("name", scenarios.ALL)
-def test_graph_edges_and_normal_equations_bit_equal(oracle, name):
+def test_graph_edges_and_normal_equations_bit_equal(oracle, pins, name):
     """buildGraph + computeActiveErrors + buildSystem: every active edge (dimension, vertex ids, error, information,
     Jacobian) and the assembled H / b / chi2, for obstacle weight multipliers 1 and 4"""
     p, hb = scenarios.scenario(name)
@@ -91,17 +88,16 @@ def test_graph_edges_and_normal_equations_bit_equal(oracle, name):
         kw = scenarios.band_kwargs(hb, b)
         for wm in (1.0, 4.0):
             Ho, bo, co = oracle.build_system(p, hb.poses[b], n, weight_multiplier=wm, jac_mode=oracle.JAC_G2O, **kw)
-            Hr, br, cr, er = rb.build_system(p, hb.poses[b], n, weight_multiplier=wm, want_edges=True, **kw)
             eo = oracle.dump_edges(p, hb.poses[b], n, weight_multiplier=wm, jac_mode=oracle.JAC_G2O, **kw)
-            assert eo.shape == er.shape, (name, b, eo.shape, er.shape)
-            assert np.array_equal(eo[:, :8], er[:, :8]), "errors / information differ"
-            assert np.array_equal(eo[:, 53:], er[:, 53:]), "graph structure differs"
-            assert np.array_equal(eo, er), "Jacobians differ"
-            assert np.array_equal(Ho, Hr) and np.array_equal(bo, br) and co == cr
+            ref = functools.cache(lambda: rb.build_system(p, hb.poses[b], n, weight_multiplier=wm, want_edges=True, **kw))
+            pins.equal(lambda: ref()[3][:, :8], eo[:, :8], (name, b, wm, "errors / information"))
+            pins.equal(lambda: ref()[3][:, 53:], eo[:, 53:], (name, b, wm, "graph structure"))
+            pins.equal(lambda: ref()[3], eo, (name, b, wm, "Jacobians"))
+            pins.equal(lambda: ref()[:3], (Ho, bo, co), (name, b, wm, "H / b / chi2"))
 
 
 @pytest.mark.parametrize("name", scenarios.ALL)
-def test_optimize_teb_bit_equal(oracle, name):
+def test_optimize_teb_bit_equal(oracle, pins, name):
     """whole optimizeTEB calls (outer x inner LM iterations, autoResize, weight adaptation, cost): poses, n, cost and
     the number of LM trials of the reference's code and of the restatement are identical"""
     p, hb = scenarios.scenario(name)
@@ -111,30 +107,34 @@ def test_optimize_teb_bit_equal(oracle, name):
         n = int(hb.n[b])
         kw = scenarios.band_kwargs(hb, b)
         ro, co, so = oracle.optimize_band(p, hb.poses[b], n, args=args, jac_mode=oracle.JAC_G2O, n_cap=hb.n_cap, **kw)
-        rr, cr, sr, ok = rb.optimize_band(p, hb.poses[b], n, args=args, n_cap=hb.n_cap, **kw)
-        assert ok and len(ro) == len(rr), (name, b, len(ro), len(rr))
-        assert np.array_equal(ro, rr), (name, b, np.abs(ro - rr).max())
-        assert co == cr
-        assert so.lm_trials == sr["lm_trials"] and so.rejected == sr["rejected"]
-        assert bool(so.status & abi.TEB_STATUS_TERMINATED) == sr["terminated"]
+        pins.equal(lambda: _optimized(rb.optimize_band(p, hb.poses[b], n, args=args, n_cap=hb.n_cap, **kw)),
+                   (True, ro, co, so.lm_trials, so.rejected, bool(so.status & abi.TEB_STATUS_TERMINATED)), (name, b))
 
 
-def test_optimize_teb_alternative_time_cost_and_disabled(oracle):
+def _optimized(res):
+    """the parts of the reference's optimizeTEB result the oracle's must equal: ok, band, cost, LM trials / rejections,
+    termination"""
+    rr, cr, sr, ok = res
+    return ok, rr, cr, sr["lm_trials"], sr["rejected"], sr["terminated"]
+
+
+def test_optimize_teb_alternative_time_cost_and_disabled(oracle, pins):
     p, hb = scenarios.scenario("C2")
     kw = scenarios.band_kwargs(hb, 0)
     args = abi.make_args(3, 2, True, 7.0, 3.0, True)
     ro, co, so = oracle.optimize_band(p, hb.poses[0], int(hb.n[0]), args=args, jac_mode=oracle.JAC_G2O, **kw)
-    rr, cr, sr, ok = rb.optimize_band(p, hb.poses[0], int(hb.n[0]), args=args, **kw)
-    assert ok and np.array_equal(ro, rr) and co == cr
+    ok_band_cost = lambda r: (r[3], r[0], r[1])
+    pins.equal(lambda: ok_band_cost(rb.optimize_band(p, hb.poses[0], int(hb.n[0]), args=args, **kw)), (True, ro, co))
     p.optimization_activate = 0        # optimizeTEB returns false before touching anything (optimal_planner.cpp:185)
-    rr, cr, sr, ok = rb.optimize_band(p, hb.poses[0], int(hb.n[0]), args=args, **kw)
     ro, co, so = oracle.optimize_band(p, hb.poses[0], int(hb.n[0]), args=args, jac_mode=oracle.JAC_G2O, **kw)
     # (isOptimized() is not checked: the constructor used here leaves optimized_ uninitialised, optimal_planner.cpp:67-70)
-    assert not ok and np.array_equal(rr, hb.poses[0][:hb.n[0]]) and np.array_equal(ro, rr)
+    pins.equal(lambda: ok_band_cost(rb.optimize_band(p, hb.poses[0], int(hb.n[0]), args=args, **kw))[:2],
+               (False, hb.poses[0][:hb.n[0]]))
+    assert np.array_equal(ro, hb.poses[0][:hb.n[0]])
     assert not (so.status & abi.TEB_STATUS_OPTIMIZED)
 
 
-def test_divergence_detection_matches(oracle):
+def test_divergence_detection_matches(oracle, pins):
     """hasDiverged (optimal_planner.cpp:1023-1039): chi2 of the final state vs divergence_detection_max_chi_squared"""
     p, hb = scenarios.scenario("divergence")
     args = abi.make_args(5, 4, True, 100.0, 1.0, False)
@@ -144,14 +144,15 @@ def test_divergence_detection_matches(oracle):
         for b in range(hb.B):
             kw = scenarios.band_kwargs(hb, b)
             ro, co, so = oracle.optimize_band(p, hb.poses[b], int(hb.n[b]), args=args, jac_mode=oracle.JAC_G2O, **kw)
-            rr, cr, sr, ok = rb.optimize_band(p, hb.poses[b], int(hb.n[b]), args=args, **kw)
-            assert np.array_equal(ro, rr) and co == cr
-            assert sr["diverged"] == (so.chi2_final > thr)
-            seen.add(sr["diverged"])
+            ref = functools.cache(lambda: rb.optimize_band(p, hb.poses[b], int(hb.n[b]), args=args, **kw))
+            pins.equal(lambda: ref()[:2], (ro, co), (thr, b))
+            diverged = bool(pins.value(lambda: ref()[2]["diverged"])[0])
+            assert diverged == (so.chi2_final > thr)
+            seen.add(diverged)
     assert seen == {True, False}
 
 
-def test_compute_cost_outside_optimize_is_undefined_in_the_reference(oracle):
+def test_compute_cost_outside_optimize_is_undefined_in_the_reference(oracle, pins):
     """computeCurrentCost on a FRESH graph (optimal_planner.cpp:1045-1051, the path HomotopyClassPlanner::
     computeCurrentCost takes): buildGraph + initializeOptimization never evaluate an edge and computeInitialGuess does
     nothing for TEB edges, so edge->chi2() reads the `_error` members as constructed. Upstream g2o leaves them
@@ -162,8 +163,9 @@ def test_compute_cost_outside_optimize_is_undefined_in_the_reference(oracle):
     p, hb = scenarios.scenario("C2")
     kw = scenarios.band_kwargs(hb, 0)
     n = int(hb.n[0])
-    assert rb.compute_cost(p, hb.poses[0], n, args=abi.make_args(5, 4, True, 50.0, 2.5, False), **kw) == 0.0
-    alt = rb.compute_cost(p, hb.poses[0], n, args=abi.make_args(5, 4, True, 50.0, 2.5, True), **kw)
+    plain, alt = pins.value(lambda: [rb.compute_cost(p, hb.poses[0], n, args=abi.make_args(5, 4, True, 50.0, 2.5, alt_time), **kw)
+                                     for alt_time in (False, True)])
+    assert plain == 0.0
     t = 0.0
     for i in range(n - 1):              # getSumOfAllTimeDiffs (timed_elastic_band.cpp:184-192), same summation order
         t += hb.poses[0][i, 3]
@@ -190,7 +192,7 @@ def _cost_from_oracle(oracle, p, hb, b, args):
 
 
 @pytest.mark.parametrize("case", ["large_at_end", "small_at_end", "middle_and_end"])
-def test_autoresize_reference_gtests_on_reference_code(oracle, teblib, case):
+def test_autoresize_reference_gtests_on_reference_code(oracle, teblib, pins, case):
     """test/teb_basics.cpp:5-68 (the reference's own gtests): same inputs, same assertions, executed on the reference's
     TimedElasticBand; the restatement and the product's host routine must return the identical band"""
     dt, hyst = 0.1, 0.1 / 3.0
@@ -206,7 +208,7 @@ def test_autoresize_reference_gtests_on_reference_code(oracle, teblib, case):
     rec = np.zeros((64, 4))
     rec[:n, 0] = np.arange(n)
     rec[:n - 1, 3] = dts
-    out = rb.auto_resize(rec, n, dt, hyst, 3, 100, False, n_cap=64)
+    out = pins.value(lambda: rb.auto_resize(rec, n, dt, hyst, 3, 100, False, n_cap=64))[0]
     d = out[:-1, 3]
     assert np.all(d <= dt + hyst + 1e-3) and np.all(dt - hyst - 1e-3 <= d)     # ASSERT_LE pairs of the gtest
     assert np.array_equal(out, oracle.auto_resize(rec, n, dt, hyst, 3, 100, False, n_cap=64))
@@ -215,18 +217,7 @@ def test_autoresize_reference_gtests_on_reference_code(oracle, teblib, case):
     assert nn == len(out) and np.array_equal(mine[:nn], out)
 
 
-def test_autoresize_random_bit_equal(oracle):
-    rng = np.random.default_rng(2)
-    for k in range(300):
-        n = int(rng.integers(3, 40))
-        rec = np.zeros((n, 4))
-        rec[:, 0] = np.cumsum(rng.uniform(0.0, 0.3, n))
-        rec[:, 1] = rng.normal(0, 0.5, n)
-        rec[:, 2] = rng.uniform(-3.2, 3.2, n)
-        rec[:n - 1, 3] = rng.choice([0.05, 0.1, 0.29, 0.3, 0.41, 0.8, 1.5], n - 1) * rng.uniform(0.9, 1.1, n - 1)
-        fast = bool(k % 2)
-        a = rb.auto_resize(rec, n, 0.3, 0.1, int(rng.integers(3, 6)) if k % 3 else 3, int(rng.choice([12, 50, 500])), fast, n_cap=1024)
-    # the same sequence again for both implementations (rng consumed identically above would hide argument differences)
+def test_autoresize_random_bit_equal(oracle, pins):
     rng = np.random.default_rng(2)
     for k in range(300):
         n = int(rng.integers(3, 40))
@@ -238,19 +229,11 @@ def test_autoresize_random_bit_equal(oracle):
         fast = bool(k % 2)
         mn = int(rng.integers(3, 6)) if k % 3 else 3
         mx = int(rng.choice([12, 50, 500]))
-        a = rb.auto_resize(rec, n, 0.3, 0.1, mn, mx, fast, n_cap=1024)
         c = oracle.auto_resize(rec, n, 0.3, 0.1, mn, mx, fast, n_cap=1024)
-        assert a.shape == c.shape and np.array_equal(a, c), k
+        pins.equal(lambda: rb.auto_resize(rec, n, 0.3, 0.1, mn, mx, fast, n_cap=1024), c, k)
 
 
-def test_init_trajectory_bit_equal(oracle):
-    rng = np.random.default_rng(4)
-    for k in range(100):
-        start = np.array([rng.normal(0, 2), rng.normal(0, 2), rng.uniform(-3, 3)])
-        goal = start + np.array([rng.normal(0, 3), rng.normal(0, 3), rng.uniform(-1, 1)])
-        diststep = float(rng.choice([0.0, 0.1, 0.35]))
-        back = bool(k % 4 == 0)
-        a = rb.init_trajectory(start, goal, diststep, 0.4, int(rng.integers(3, 8)) if k % 2 else 3, back, n_cap=2048)
+def test_init_trajectory_bit_equal(oracle, pins):
     rng = np.random.default_rng(4)
     for k in range(100):
         start = np.array([rng.normal(0, 2), rng.normal(0, 2), rng.uniform(-3, 3)])
@@ -258,22 +241,27 @@ def test_init_trajectory_bit_equal(oracle):
         diststep = float(rng.choice([0.0, 0.1, 0.35]))
         back = bool(k % 4 == 0)
         ms = int(rng.integers(3, 8)) if k % 2 else 3
-        a = rb.init_trajectory(start, goal, diststep, 0.4, ms, back, n_cap=2048)
         c = oracle.init_trajectory(start, goal, diststep, 0.4, ms, back, n_cap=2048)
-        assert a.shape == c.shape and np.array_equal(a, c), k
+        pins.equal(lambda: rb.init_trajectory(start, goal, diststep, 0.4, ms, back, n_cap=2048), c, k)
 
 
-def test_golden_reference_vectors_are_current():
-    """the committed fixture was generated from THIS reference build: regenerate a slice and compare"""
+def test_golden_reference_vectors_are_current(pins):
+    """the committed fixture was generated from the reference build the other pins come from: a slice regenerated from
+    that build equals the fixture"""
     from tests.golden import make_golden_ref
     z = np.load(GOLDEN_REF, allow_pickle=False)
-    fresh = make_golden_ref.generate(only=("C1", "via_ordered"))
-    for k, v in fresh.items():
-        assert np.array_equal(z[k], v), k
+    only = ("C1", "via_ordered")
+    keys = [k for k in z.files if k.split("/")[0] in only]
+
+    def fresh():
+        f = make_golden_ref.generate(only=only)
+        assert sorted(f) == sorted(keys)
+        return [f[k] for k in keys]
+    pins.equal(fresh, [z[k] for k in keys])
 
 
 @pytest.mark.parametrize("cfg", ["C1", "C2", "C3", "C4"])
-def test_h_signatures_match_the_reference_header(oracle, cfg):
+def test_h_signatures_match_the_reference_header(oracle, pins, cfg):
     """calculateEquivalenceClass executed by the reference's own h_signature.h (HSignature: long double complex
     accumulation; HSignature3d: numeric integration over the x-y-t obstacle 'conductors', with and without the band's
     time differences) against the oracle restatement, plus isValid / isReasonable and the class comparison the planner
@@ -285,14 +273,15 @@ def test_h_signatures_match_the_reference_header(oracle, cfg):
     for b in range(hb.B):
         rec, n = hb.poses[b], int(hb.n[b])
         p.include_dynamic_obstacles = 0
-        want, valid, reasonable = rb.h_signature(p, rec, n, obst)
+        want, valid, reasonable = pins.value(lambda: rb.h_signature(p, rec, n, obst))
+        want = complex(*want)
         got = oracle.h_signature(p, rec, n, obst)
         assert valid and np.isfinite(want.real) and np.isfinite(want.imag)
         assert abs(got - want) <= 1e-15 * max(1.0, abs(want)), (cfg, b, got, want)
         sig2.append((got, want))
         p.include_dynamic_obstacles = 1
         for use_dt in (True, False):
-            want3, valid3, reasonable3 = rb.h_signature(p, rec, n, obst, use_timediffs=use_dt)
+            want3, valid3, reasonable3 = pins.value(lambda: rb.h_signature(p, rec, n, obst, use_timediffs=use_dt))
             got3 = oracle.h_signature(p, rec, n, obst, use_timediffs=use_dt)
             assert valid3
             assert np.array_equal(got3, want3), (cfg, b, use_dt, np.abs(got3 - want3).max())
@@ -308,11 +297,12 @@ def test_h_signatures_match_the_reference_header(oracle, cfg):
     for name, pp, hbb in make_golden.hsig_cases():
         ob = hbb.obstacles[0][:hbb.obst_count[0]]
         for b in range(hbb.B):
-            want, _, _ = rb.h_signature(pp, hbb.poses[b], hbb.n[b], ob)
+            want = pins.value(lambda: rb.h_signature(pp, hbb.poses[b], hbb.n[b], ob))[0]
             have = g[name][b]
             if pp.include_dynamic_obstacles:
                 assert np.array_equal(want, have[:len(ob)])
             else:
+                want = complex(*want)
                 assert abs(want - complex(have[0], have[1])) <= 1e-15 * max(1.0, abs(want))
 
 
@@ -345,7 +335,7 @@ def _explorer_inputs(rng, n_obst, dynamic):
 
 @pytest.mark.parametrize("prm", [False, True])
 @pytest.mark.parametrize("dynamic", [0, 1])
-def test_candidate_exploration_matches_the_reference_planner(oracle, prm, dynamic):
+def test_candidate_exploration_matches_the_reference_planner(oracle, pins, prm, dynamic):
     """exploreEquivalenceClassesAndInitTebs of the reference's own HomotopyClassPlanner / graph_search.cpp (key-point graph
     and probabilistic roadmap, DepthFirst enumeration order, addAndInitNewTeb with the path variant of
     initTrajectoryToGoal, H-signature filtering with both signature kinds, class budget) against the sequential
@@ -364,7 +354,9 @@ def test_candidate_exploration_matches_the_reference_planner(oracle, prm, dynami
         start = [-4.0, rng.uniform(-0.5, 0.5), rng.uniform(-0.4, 0.4)]
         goal = [4.0, rng.uniform(-0.5, 0.5), rng.uniform(-0.4, 0.4)]
         cycles = 2
-        want = rb.hcp_explore(p, hcp, start, goal, rows, pool, cycles=cycles, prm=prm)
+        counts, *bands = pins.value(lambda: _flat_explore(rb.hcp_explore(p, hcp, start, goal, rows, pool, cycles=cycles, prm=prm)))
+        ends = np.cumsum(counts).astype(int)
+        want = [bands[e - int(k):e] for k, e in zip(counts, ends)]
         ex = X.Explorer(p, hcp, oracle, rows, obstacles)
         for c in range(cycles):
             ex.classes, ex.tebs = [], []
@@ -375,8 +367,27 @@ def test_candidate_exploration_matches_the_reference_planner(oracle, prm, dynami
                 assert np.abs(got - ref).max() < 1e-12, (case, c, k, np.abs(got - ref).max())
 
 
+def _flat_explore(res):
+    """hcp_explore's result (per cycle a list of bands) as [candidates per cycle, band, band, ...]"""
+    return [np.array([len(c) for c in res])] + [band for c in res for band in c]
+
+
+def _flat_plan(res):
+    """hcp_plan's result as ([(ok, best, candidates), costs] per cycle, [band, band, ...])"""
+    return ([x for ok, best, cands in res for x in (np.array([ok, best, len(cands)]), np.array([c for c, _ in cands]))],
+            [band for _, _, cands in res for _, band in cands])
+
+
+def _unflat_plan(heads, bands):
+    res = []
+    for (ok, best, k), costs in zip(heads[0::2], heads[1::2]):
+        res.append((bool(ok), int(best), list(zip(costs.tolist(), bands[:int(k)]))))
+        bands = bands[int(k):]
+    return res
+
+
 @pytest.mark.parametrize("prm", [False, True])
-def test_planning_cycles_match_the_reference_planner(oracle, teblib, prm):
+def test_planning_cycles_match_the_reference_planner(oracle, teblib, pins, prm):
     """consecutive HomotopyClassPlanner::plan(start, goal) calls of the reference's own planner (updateAllTEBs,
     renewAndAnalyzeOldTebs, deletePlansDetouringBackwards, graph exploration, optimizeAllTEBs, selectBestTeb) against the
     sequential restatement oracle/hcp_explore.py::Planner with the start pose moving along: same number of candidates,
@@ -397,7 +408,10 @@ def test_planning_cycles_match_the_reference_planner(oracle, teblib, prm):
                "roadmap_graph_area_width": 5.0, "roadmap_graph_area_length_scale": 1.0, "roadmap_graph_no_samples": 10}
         goal = [4.0, rng.uniform(-0.3, 0.3), rng.uniform(-0.2, 0.2)]
         starts = [[-4.0 + 0.2 * c, 0.03 * c + rng.normal(0, 0.01), 0.05] for c in range(4)]
-        want = rb.hcp_plan(p, hcp, starts, goal, rows, pool, prm=prm)
+        ref = functools.cache(lambda: _flat_plan(rb.hcp_plan(p, hcp, starts, goal, rows, pool, prm=prm)))
+        # the bands are stored in float32: the bound below leaves room for the rounding, so that it still holds against
+        # the reference's float64 bands
+        want = _unflat_plan(pins.value(lambda: ref()[0]), pins.value(lambda: ref()[1], np.float32))
         pl = X.Planner(p, hcp, oracle, rows, obstacles, simple_exploration=not prm)
         pl.jac_mode = oracle.JAC_G2O
         pl.obst_vertices = pool
@@ -416,5 +430,5 @@ def test_planning_cycles_match_the_reference_planner(oracle, teblib, prm):
             carried_best = best >= 0
             for k, ((cost, band), rec) in enumerate(zip(cands, pl.tebs)):
                 assert band.shape == rec.shape, (case, c, k, band.shape, rec.shape)
-                assert np.abs(band - rec).max() < 1e-5, (case, c, k, np.abs(band - rec).max())
+                assert (np.abs(band - rec) + np.abs(band) * 2.0 ** -24).max() < 1e-5, (case, c, k, np.abs(band - rec).max())
                 assert abs(cost - pl.costs[k]) <= 1e-6 * max(1.0, abs(cost)), (case, c, k, cost, pl.costs[k])
