@@ -39,7 +39,8 @@ extern "C" {
 /* per-band status bits written to status[] */
 #define TEB_STATUS_OPTIMIZED       1   /* optimizeTEB returned true (optimal_planner.cpp:220)      */
 #define TEB_STATUS_TOO_FEW_POSES   2   /* sizePoses < min_samples guard (optimal_planner.cpp:377)   */
-#define TEB_STATUS_CHOL_FAILED     4   /* at least one trial factorisation hit a non-positive pivot */
+#define TEB_STATUS_CHOL_FAILED     4   /* at least one trial factorisation hit a pivot that is not a positive normal
+                                          number (<= 0, subnormal, inf or NaN); a non-finite solution is not a failure */
 #define TEB_STATUS_NONFINITE       8   /* non-finite chi2 / lambda encountered                      */
 #define TEB_STATUS_TERMINATED     16   /* LM returned Terminate in the last optimizeGraph call      */
 #define TEB_STATUS_DISABLED       32   /* optimization_activate == false / max_vel_x < 0.01          */
@@ -310,6 +311,20 @@ int64_t tebgpu_get_info(const tebgpu_ctx* ctx, int32_t which);
  * (BlockSolver::buildSystem, SURVEY §3.3 step 2). */
 int32_t tebgpu_build_system(tebgpu_ctx* ctx, const TebBatch* batch, int32_t outer_index,
                             double* Hb_out, double* chi2_out, int32_t device_ptrs);
+
+/* LM linear solve only (test entry point for the solve kernels of the default solver): for every band b and trial
+ * k < K (1 .. 8), solve (H_b + lambda_bk * I_real) dx = b_b with the mapping chosen by tebgpu_set_warp_solver (0 thread,
+ * 1 warp, 3 twisted; 2 and 4 resolve by the number of systems B * K as in optimize), where lambda_bk is lambda[b]
+ * escalated k times (lambda *= ni, ni *= 2), as the speculative rounds do. I_real is the identity on the real unknowns:
+ * rows 0 .. 2 (start pose) and 4 n - 4 .. 4 n - 1 (goal pose, dt of the last pose) are identity rows of H.
+ * Same grid, shared memory and kernel choice as round 0 of an LM iteration of tebgpu_optimize_batch.
+ * HOST buffers: Hb [B][4 n_cap][12] in the layout tebgpu_build_system writes, n [B] (3 .. n_cap), lambda [B], ni [B];
+ * outputs dx_out [B][K][4 n_cap] (rows a kernel does not write - 4 n[b] .. 4 n_cap - 1, and the whole system after a
+ * failed factorisation in modes 0 / 1 - are NaN), ok_out [B][K] (1: the factorisation succeeded, the flag the trial
+ * evaluation reads; 0: TEB_STATUS_CHOL_FAILED), lambda_out [B][K] (the damping the kernel used). */
+int32_t tebgpu_solve_system(tebgpu_ctx* ctx, int32_t B, int32_t n_cap, const int32_t* n, const double* Hb,
+                            const double* lambda, const double* ni, int32_t K,
+                            double* dx_out, int32_t* ok_out, double* lambda_out);
 
 /* TebOptimalPlanner::computeCurrentCost called OUTSIDE optimizeTEB (optimal_planner.cpp:1041-1094, graph rebuilt with
  * weight multiplier 1, errors evaluated at the current state): HOST buffers; writes cost[], chi2[], status[]. */

@@ -80,6 +80,8 @@ def load_library(build_if_missing=False):
     L.tebgpu_h_signature.argtypes = [vp, C.POINTER(abi.TebBatch), C.c_int32, vp, C.c_int32]
     L.tebgpu_build_system.restype = C.c_int32
     L.tebgpu_build_system.argtypes = [vp, C.POINTER(abi.TebBatch), C.c_int32, vp, vp, C.c_int32]
+    L.tebgpu_solve_system.restype = C.c_int32
+    L.tebgpu_solve_system.argtypes = [vp, C.c_int32, C.c_int32, vp, vp, vp, vp, C.c_int32, vp, vp, vp]
     L.tebgpu_select_best.restype = C.c_int32
     L.tebgpu_select_best.argtypes = [vp, C.c_int32, C.c_int32, C.c_int32, C.c_double, C.c_double]
     L.tebgpu_auto_resize_host.restype = C.c_int32
@@ -229,6 +231,26 @@ class TebGpu:
         self._check(self.lib.tebgpu_build_system(self.ctx, C.byref(bs), outer_index, Hb.ctypes.data, chi2.ctypes.data, 0),
                     "tebgpu_build_system")
         return Hb, chi2
+
+    def solve_system(self, Hb, n, lam, ni, K):
+        """LM linear solve only, with the mapping chosen by set_warp_solver: Hb [B][4*n_cap][12] (build_system's
+        layout), n [B], lam / ni [B] (damping state before trial 0), K trials per band.
+        Returns (dx [B][K][4*n_cap], ok [B][K], lam_used [B][K])."""
+        import numpy as np
+        Hb = np.ascontiguousarray(Hb, dtype=np.float64)
+        B, rows = Hb.shape[0], Hb.shape[1]
+        if Hb.shape[2] != 12 or rows % 4:
+            raise ValueError(f"Hb must be [B][4*n_cap][12], got {Hb.shape}")
+        n = np.ascontiguousarray(n, dtype=np.int32)
+        lam = np.ascontiguousarray(np.broadcast_to(lam, (B,)), dtype=np.float64)
+        ni = np.ascontiguousarray(np.broadcast_to(ni, (B,)), dtype=np.float64)
+        dx = np.empty((B, K, rows))
+        ok = np.empty((B, K), dtype=np.int32)
+        lam_used = np.empty((B, K))
+        self._check(self.lib.tebgpu_solve_system(self.ctx, B, rows // 4, n.ctypes.data, Hb.ctypes.data, lam.ctypes.data,
+                                                 ni.ctypes.data, int(K), dx.ctypes.data, ok.ctypes.data,
+                                                 lam_used.ctypes.data), "tebgpu_solve_system")
+        return dx, ok, lam_used
 
     def close(self):
         if self.ctx:

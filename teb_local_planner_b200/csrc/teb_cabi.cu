@@ -488,6 +488,43 @@ static void launch_trial_eval(tebgpu_ctx* ctx, const SpecBufs& spec, const DevBa
   else k_trial_eval<2, false><<<B, 32 * K, smem, st>>>(db, kp, spec, it, round, g, tag);
 }
 
+/* The solve of one speculative round of solver 2: the B x K (band, trial) systems of round `round` of LM iteration `it`
+ * (retry-list index g), with the mapping chosen by tebgpu_set_warp_solver - in the automatic modes by the number of
+ * systems. Shared by issue_optimize and tebgpu_solve_system, so that the test entry point runs the optimizer's grid,
+ * shared-memory size and kernel choice. Returns the number of kernels launched. */
+static int launch_solve_kernel(const tebgpu_ctx* ctx, const DevBatch& db, const SpecBufs& spec, int B, int K, int it, int round,
+                               int g, cudaStream_t s) {
+  /* ring depth: 10 rows unless TEBGPU_RING asks for 20 / 30. Measured (profiles/r2_history.md): deeper rings do
+   * not shorten the chain - a lone solver warp is bound by its own fp64 issue rate (~75 DFMA per pivot at 2
+   * cycles each), not by the prefetch distance - and they cost residency (20 rows: 3 warps per SM). */
+  const int bk = B * K;
+  const int warps = (bk + 31) / 32;
+  const int ring = ctx->ring == 0 ? 10 : ctx->ring;
+  /* k_solve_warp: the sequential order spread over a warp (cross-check only) */
+  const bool warp_solver = ctx->warp_solver == 1 || (ctx->warp_solver == 2 && bk <= 148 * 8);
+  const size_t smem_lat = solve_lat_smem_bytes(db.n_cap);
+  /* automatic: while the round's systems fit LAT_WAVES waves of resident CTAs (one warp + its whole system per CTA)
+   * the twisted solver's ~0.065 ms per wave (200 poses) beats the 0.26 ms a thread-per-system solve takes
+   * regardless of the count */
+  const long long lat_wave = smem_lat <= 232448 ? 148LL * (232448 / smem_lat > 16 ? 16 : 232448 / smem_lat) : 0;
+  const bool lat_solver = lat_wave > 0 && (ctx->warp_solver == 3 || (ctx->warp_solver == 4 && bk <= LAT_WAVES * lat_wave));
+  if (lat_solver) k_solve_lat<<<bk, 32, smem_lat, s>>>(db, spec, it, round, g);
+  else if (round > 0 && ctx->warp_solver == 4 && lat_wave > 0) {
+    /* retry round of the throughput regime: both mappings are launched, the list length decides on the device */
+    SpecBufs sl = spec;
+    const long long cap = LAT_WAVES * lat_wave < bk ? LAT_WAVES * lat_wave : bk;
+    sl.lat_cap = (int32_t)cap;
+    k_solve_lat<<<(unsigned)cap, 32, smem_lat, s>>>(db, sl, it, round, g);
+    k_solve_tpb<10><<<warps, 32, tpb_ring_bytes(10), s>>>(db, sl, it, round, g);
+    return 2;
+  }
+  else if (warp_solver) k_solve_warp<<<(bk + SW_WARPS - 1) / SW_WARPS, 32 * SW_WARPS, 0, s>>>(db, spec, it, round, g);
+  else if (ring == 30) k_solve_tpb<30><<<warps, 32, tpb_ring_bytes(30), s>>>(db, spec, it, round, g);
+  else if (ring == 20) k_solve_tpb<20><<<warps, 32, tpb_ring_bytes(20), s>>>(db, spec, it, round, g);
+  else k_solve_tpb<10><<<warps, 32, tpb_ring_bytes(10), s>>>(db, spec, it, round, g);
+  return 1;
+}
+
 static KParams make_kparams(const tebgpu_ctx* ctx, const TebBatch* bt, double weight_multiplier) {
   const TebParams& p = ctx->params;
   KParams k;
@@ -671,35 +708,7 @@ static int32_t issue_optimize(tebgpu_ctx* ctx, const TebBatch* bt, const TebOpti
         const bool fork = overlap && rounds > 1 && !kp.has_vor;
         cudaStream_t rs = st;
         auto launch_solve = [&](const SpecBufs& spec, int K, int round, cudaStream_t s) {
-          /* ring depth: 10 rows unless TEBGPU_RING asks for 20 / 30. Measured (profiles/r2_history.md): deeper rings do
-           * not shorten the chain - a lone solver warp is bound by its own fp64 issue rate (~75 DFMA per pivot at 2
-           * cycles each), not by the prefetch distance - and they cost residency (20 rows: 3 warps per SM). */
-          const int bk = B * K;
-          const int warps = (bk + 31) / 32;
-          const int ring = ctx->ring == 0 ? 10 : ctx->ring;
-          /* k_solve_warp: the sequential order spread over a warp (cross-check only) */
-          const bool warp_solver = ctx->warp_solver == 1 || (ctx->warp_solver == 2 && bk <= 148 * 8);
-          const size_t smem_lat = solve_lat_smem_bytes(bt->n_cap);
-          /* automatic: while the round's systems fit LAT_WAVES waves of resident CTAs (one warp + its whole system per CTA)
-           * the twisted solver's ~0.065 ms per wave (200 poses) beats the 0.26 ms a thread-per-system solve takes
-           * regardless of the count */
-          const long long lat_wave = smem_lat <= 232448 ? 148LL * (232448 / smem_lat > 16 ? 16 : 232448 / smem_lat) : 0;
-          const bool lat_solver = lat_wave > 0 && (ctx->warp_solver == 3 || (ctx->warp_solver == 4 && bk <= LAT_WAVES * lat_wave));
-          if (lat_solver) k_solve_lat<<<bk, 32, smem_lat, s>>>(db, spec, it, round, g);
-          else if (round > 0 && ctx->warp_solver == 4 && lat_wave > 0) {
-            /* retry round of the throughput regime: both mappings are launched, the list length decides on the device */
-            SpecBufs sl = spec;
-            const long long cap = LAT_WAVES * lat_wave < bk ? LAT_WAVES * lat_wave : bk;
-            sl.lat_cap = (int32_t)cap;
-            k_solve_lat<<<(unsigned)cap, 32, smem_lat, s>>>(db, sl, it, round, g);
-            k_solve_tpb<10><<<warps, 32, tpb_ring_bytes(10), s>>>(db, sl, it, round, g);
-            ++launches;
-          }
-          else if (warp_solver) k_solve_warp<<<(bk + SW_WARPS - 1) / SW_WARPS, 32 * SW_WARPS, 0, s>>>(db, spec, it, round, g);
-          else if (ring == 30) k_solve_tpb<30><<<warps, 32, tpb_ring_bytes(30), s>>>(db, spec, it, round, g);
-          else if (ring == 20) k_solve_tpb<20><<<warps, 32, tpb_ring_bytes(20), s>>>(db, spec, it, round, g);
-          else k_solve_tpb<10><<<warps, 32, tpb_ring_bytes(10), s>>>(db, spec, it, round, g);
-          ++launches;
+          launches += launch_solve_kernel(ctx, db, spec, B, K, it, round, g, s);
         };
         for (int round = 0; round < rounds; ++round, ++g) {
           const int K = sched[round];
@@ -1090,6 +1099,58 @@ int32_t tebgpu_build_system(tebgpu_ctx* ctx, const TebBatch* bt, int32_t outer_i
     delete[] hn;
   }
   CUDA_TRY(ctx, cudaStreamSynchronize(st));
+  return TEBGPU_OK;
+}
+
+int32_t tebgpu_solve_system(tebgpu_ctx* ctx, int32_t B, int32_t n_cap, const int32_t* n, const double* Hb, const double* lambda,
+                            const double* ni, int32_t K, double* dx_out, int32_t* ok_out, double* lambda_out) {
+  if (!ctx || !n || !Hb || !lambda || !ni || !dx_out || !ok_out || !lambda_out) return TEBGPU_ERR_INVALID_ARG;
+  if (B < 1 || n_cap < 3 || K < 1 || K > SPEC_K_MAX) { ctx->err = "bad solve dimensions"; return TEBGPU_ERR_INVALID_ARG; }
+  if (B > ctx->lim.max_bands || n_cap > ctx->lim.max_poses) { ctx->err = "solve exceeds the context limits"; return TEBGPU_ERR_CAPACITY; }
+  for (int b = 0; b < B; ++b)
+    if (n[b] < 3 || n[b] > n_cap) { ctx->err = "n[b] outside 3 .. n_cap"; return TEBGPU_ERR_INVALID_ARG; }
+  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  cudaStream_t st = ctx->stream;
+  const size_t rows = (size_t)4 * n_cap;
+  std::vector<BandState> hs((size_t)B);
+  for (int b = 0; b < B; ++b) {
+    std::memset(&hs[b], 0, sizeof(BandState));
+    hs[b].active = 1;
+    hs[b].lambda = lambda[b];
+    hs[b].ni = ni[b];
+  }
+  CUDA_TRY(ctx, cudaMemcpyAsync(ctx->Hb, Hb, (size_t)B * rows * HROW * sizeof(double), cudaMemcpyHostToDevice, st));
+  CUDA_TRY(ctx, cudaMemcpyAsync(ctx->d_n, n, (size_t)B * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+  CUDA_TRY(ctx, cudaMemcpyAsync(ctx->state, hs.data(), (size_t)B * sizeof(BandState), cudaMemcpyHostToDevice, st));
+  DevBatch db;
+  std::memset(&db, 0, sizeof(db));
+  db.B = B; db.n_cap = n_cap; db.n = ctx->d_n; db.Hb = ctx->Hb; db.state = ctx->state;
+  db.tile = KA2_TP; db.chunks = (n_cap + KA2_TP - 1) / KA2_TP; db.dmax_parts = ctx->dmax_parts; db.defer = ctx->defer;
+  SpecBufs spec = ctx->spec; /* round 0, no selection list: system t = K b + k */
+  spec.K = K; spec.sel_list = nullptr; spec.sel_cnt = nullptr; spec.defer = nullptr; spec.skip_tag = 0; spec.lat_cap = 0;
+  /* the solution scratch is filled with NaN first: rows a kernel does not write (4 n[b] .. 4 n_cap - 1, and the whole
+   * system after a failed factorisation in the modes that stop there) come back as NaN */
+  const int warps = (B * K + 31) / 32;
+  const size_t dx_elems = (size_t)warps * 32 * rows;
+  CUDA_TRY(ctx, cudaMemsetAsync(spec.dx, 0xff, dx_elems * sizeof(double), st));
+  CUDA_TRY(ctx, cudaMemsetAsync(spec.res, 0, (size_t)B * SPEC_K_MAX * RES_STRIDE * sizeof(double), st));
+  ctx->launches = launch_solve_kernel(ctx, db, spec, B, K, /*it=*/1, /*round=*/0, /*g=*/0, st);
+  CUDA_TRY(ctx, cudaGetLastError());
+  std::vector<double> hdx(dx_elems), hres((size_t)B * SPEC_K_MAX * RES_STRIDE);
+  CUDA_TRY(ctx, cudaMemcpyAsync(hdx.data(), spec.dx, dx_elems * sizeof(double), cudaMemcpyDeviceToHost, st));
+  CUDA_TRY(ctx, cudaMemcpyAsync(hres.data(), spec.res, hres.size() * sizeof(double), cudaMemcpyDeviceToHost, st));
+  CUDA_TRY(ctx, cudaStreamSynchronize(st));
+  /* de-interleave: system t = K b + k sits in lane t & 31 of solver warp t >> 5, row r at [r][lane] */
+  for (int b = 0; b < B; ++b)
+    for (int k = 0; k < K; ++k) {
+      const size_t t = (size_t)K * b + k;
+      const double* src = hdx.data() + (t >> 5) * 32 * rows + (t & 31);
+      double* dst = dx_out + t * rows;
+      for (size_t r = 0; r < rows; ++r) dst[r] = src[r * 32];
+      const double* res = hres.data() + ((size_t)b * SPEC_K_MAX + k) * RES_STRIDE;
+      ok_out[t] = res[5] != 0.0 ? 1 : 0;
+      lambda_out[t] = res[6];
+    }
   return TEBGPU_OK;
 }
 

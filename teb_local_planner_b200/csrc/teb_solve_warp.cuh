@@ -103,7 +103,7 @@ __global__ void __launch_bounds__(32 * SW_WARPS) k_solve_warp(DevBatch db, SpecB
     }
     __syncwarp();
     const double d = cb[0];
-    if (!(d > 0) || !isfinite(d)) ok = false;
+    if (!pivot_ok(d)) ok = false;
     const double inv = 1.0 / d;
     const double yj = cb[11];
     const int uC = (m - s) & 15;

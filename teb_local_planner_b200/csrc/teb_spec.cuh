@@ -66,6 +66,14 @@ __device__ __forceinline__ int spec_band(const DevBatch& db, const SpecBufs& sp,
   return slot;
 }
 
+/* Failure contract of the LM linear solve, shared by every mapping of solver 2 (k_solve_tpb, k_solve_warp, k_solve_lat):
+ * a factorisation FAILS - res[5] = 0, TEB_STATUS_CHOL_FAILED, and the trial evaluation takes dx = b as
+ * LinearSolverCSparse leaves it - iff some pivot d of the LDL^T is not a positive normal number: d <= 0 (CSparse's "not
+ * positive definite", cs_chol stops at d <= 0), NaN, infinite, or subnormal (its reciprocal overflows, and the fast
+ * reciprocal of k_solve_lat flushes it to zero). Nothing else fails: a non-finite SOLUTION from valid pivots is reported
+ * as a success, as CSparse does, and the non-finite chi2 of that trial ends the LM iteration as it does in g2o. */
+__device__ __forceinline__ bool pivot_ok(double d) { return d >= 2.2250738585072014e-308 && isfinite(d); }
+
 /* lambda / nu of trial q0 + k given the state before trial q0 (only rejections in between) */
 __device__ __forceinline__ void spec_lambda(double& lambda, double& ni, int k) {
   for (int t = 0; t < k; ++t) { lambda *= ni; ni *= 2; }
@@ -163,7 +171,7 @@ __global__ void __launch_bounds__(32) k_solve_tpb(DevBatch db, SpecBufs sp, int 
     for (int s = 0; s < 11; ++s) {
       const int j = j0 + s;
       const double d = E[0][s];
-      if (!(d > 0) || !isfinite(d)) ok = false;
+      if (!pivot_ok(d)) ok = false;
       const double inv = 1.0 / d;
       const double yj = Y[s];
       double cu[11];
